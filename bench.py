@@ -17,6 +17,14 @@ Workload (BASELINE.json config 3): 6 views, 512x512x256 float32, 41^3 PSFs,
 
 N > 1: independent volumes (blocks) sharded one per rank, no collective on the
 data path (SURVEY.md §8e) -- "weak" scaling.
+
+--dump-outputs DIR (rank 0) writes what the last timed step of each timed path handed back, so that two builds can
+be compared output for output on the same seeded inputs:
+  psi.npy             psi of the device-resident loop after the last timed step
+  e2e_psi.npy         psi returned by the last timed e2e call with pageable host buffers
+  e2e_pinned_psi.npy  the same with page-locked host buffers
+float32, each the whole volume when it has at most DUMP_VOXELS voxels, else the voxels at DUMP_SEED's fixed sample of
+flat indices (sorted); at most 3 x 16 MiB in all.
 """
 from __future__ import annotations
 
@@ -41,6 +49,8 @@ LAMBDA = 0.006
 MIN_VALUE = 1e-4
 METRIC = "rl_deconv_gvoxel_view_iter_per_s"
 UNIT = "Gvoxel*view*iter/s"
+DUMP_VOXELS = 1 << 22
+DUMP_SEED = 20240607
 
 
 def parse():
@@ -61,7 +71,23 @@ def parse():
     ap.add_argument("--blocks", type=int, default=64)
     ap.add_argument("--no-extra", action="store_true",
                     help="skip the config-4 / config-5 sub-records of the default run (blocks batch, 1024^3 volume)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (native deconv workload only)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and (args.impl != "native" or args.workload != "deconv"):
+        ap.error("--dump-outputs needs --impl native and --workload deconv")
+    return args
+
+
+def dump_sample(a):
+    """`a` itself when it is small enough, else its voxels at a fixed seeded sample of flat indices."""
+    flat = np.ascontiguousarray(a).reshape(-1)
+    if flat.size <= DUMP_VOXELS:
+        return np.array(a, copy=True)
+    idx = np.sort(np.random.default_rng(DUMP_SEED).choice(flat.size, DUMP_VOXELS, replace=False))
+    return flat[idx]
 
 
 def peaks():
@@ -286,6 +312,9 @@ def main():
     barrier()
     wall_ms = (time.perf_counter() - t_wall0) * 1e3
     clocks = sampler.stop()
+    outputs = {}
+    if args.dump_outputs and rank == 0:
+        outputs["psi"] = dump_sample(plan.get_psi())
     dev_ms = max_over_ranks(dev_ms)
     units_per_rank = nvox * args.views * args.iterations * args.steps
     value = world * units_per_rank / (dev_ms * 1e-3) / 1e9
@@ -346,8 +375,12 @@ def main():
         pinned_s = measure(data["views"], data["weights"], psi_host)
         pageable_views = [np.array(a, copy=True) for a in data["views"]]      # plain malloc'ed numpy memory
         pageable_weights = [np.array(a, copy=True) for a in data["weights"]]
-        pageable_s = measure(pageable_views, pageable_weights, np.array(data["psi0"], copy=True))
+        pageable_psi = np.array(data["psi0"], copy=True)
+        pageable_s = measure(pageable_views, pageable_weights, pageable_psi)
         del pageable_views, pageable_weights
+        if args.dump_outputs and rank == 0:
+            outputs["e2e_psi"] = dump_sample(pageable_psi)
+            outputs["e2e_pinned_psi"] = dump_sample(psi_host)
         e2e = {"value": world * units_per_rank / pageable_s / 1e9, "unit": UNIT,
                "h2d_bytes_per_step": int((2 * args.views + 1) * nvox * 4 + ksz * 4), "d2h_bytes_per_step": int(nvox * 4),
                "ms_per_step": pageable_s / args.steps * 1e3,
@@ -398,6 +431,10 @@ def main():
             "wall_ms_timed_region": wall_ms, "roofline": roofline, "cpu_baseline": cpu_baseline,
             "config4": config4, "config5": config5,
         }
+        if args.dump_outputs and rank == 0:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, a in outputs.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
         print(json.dumps(line))
     if dist is not None:
         dist.destroy_process_group()

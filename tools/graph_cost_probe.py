@@ -1,5 +1,5 @@
 import sys, time, os
-sys.path.insert(0, '/root/repo')
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
 from libmultiviewnative_b200 import load
 lib = load()
