@@ -184,6 +184,11 @@ LMVN_EXPORT int lmvn_dist_buffer(lmvn_dist* plan, int which, void** device_ptr, 
  * spectrum = nz*ny*(nx/2+1) interleaved (re,im) pairs.  c2r is unnormalised. */
 LMVN_EXPORT int lmvn_debug_rfftn(const float* in, const int* dims_zyx, float* spectrum, int device);
 LMVN_EXPORT int lmvn_debug_irfftn(const float* spectrum, const int* dims_zyx, float* out, int device);
+/* Sets every byte of every arena parked for later handles (what lmvn_release_cached_memory frees), on every device, to
+ * `byte` and waits for it:
+ * the next handle that takes one starts on memory full of that pattern (0xff: NaN, 0x3f: about 0.75), so that a read
+ * of a buffer the call did not write shows up in its result. */
+LMVN_EXPORT int lmvn_debug_fill_parked_arenas(int byte);
 
 #ifdef __cplusplus
 }

@@ -73,6 +73,7 @@ EXTENSION_SYMBOLS = [
     "lmvn_last_geometry",
     "lmvn_plan_destroy", "lmvn_plan_get_info", "lmvn_plan_set_view", "lmvn_plan_set_psi", "lmvn_plan_get_psi",
     "lmvn_plan_iterate", "lmvn_plan_convolve", "lmvn_plan_profile", "lmvn_plan_synchronize", "lmvn_debug_rfftn", "lmvn_debug_irfftn",
+    "lmvn_debug_fill_parked_arenas",
     "lmvn_dist_create", "lmvn_dist_destroy", "lmvn_dist_get_info", "lmvn_dist_export_handle", "lmvn_dist_connect_ipc",
     "lmvn_dist_connect_local", "lmvn_dist_set_view_slab", "lmvn_dist_set_psi_slab", "lmvn_dist_get_psi_slab",
     "lmvn_dist_psf_phase", "lmvn_dist_conv_phase", "lmvn_dist_barrier", "lmvn_dist_reset_barrier", "lmvn_dist_iterate",
@@ -177,6 +178,7 @@ class Library:
         L.lmvn_dist_buffer.argtypes = [C.c_void_p, C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_ulonglong)]
         L.lmvn_debug_rfftn.argtypes = [c_float_p, c_int_p, c_float_p, C.c_int]
         L.lmvn_debug_irfftn.argtypes = [c_float_p, c_int_p, c_float_p, C.c_int]
+        L.lmvn_debug_fill_parked_arenas.argtypes = [C.c_int]
 
     def set_padding(self, mode: int):
         """0: circular at the image extents (the CPU path, default); 1: zero_padd (the reference's GPU geometry)."""
@@ -188,6 +190,10 @@ class Library:
 
     def release_cached_memory(self):
         self.lib.lmvn_release_cached_memory()
+
+    def fill_parked_arenas(self, byte: int):
+        """Sets every byte of the arenas parked for later calls to `byte` (tests: the next call runs on dirty memory)."""
+        self._check(self.lib.lmvn_debug_fill_parked_arenas(int(byte)), "lmvn_debug_fill_parked_arenas")
 
     # -- error plumbing ----------------------------------------------------
     def last_error(self) -> str:

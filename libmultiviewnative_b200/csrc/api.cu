@@ -246,6 +246,9 @@ extern "C" int lmvn_debug_rfftn(const float* in, const int* dims_zyx, float* spe
 extern "C" int lmvn_debug_irfftn(const float* spectrum, const int* dims_zyx, float* out, int device) {
   return lmvn::debug_transform(spectrum, dims_zyx, out, device, true);
 }
+extern "C" int lmvn_debug_fill_parked_arenas(int byte) {
+  return lmvn::debug_fill_parked_arenas(byte);
+}
 
 // ---------------------------------------------------------------------------------
 // reference C API: GPU entry points (ref: src/multiviewnative.cu:58-142)

@@ -345,6 +345,19 @@ void release_cached_memory() {
   g_parked.clear();
 }
 
+int debug_fill_parked_arenas(int byte) {
+  int prev = 0;
+  LMVN_CUDA_TRY(cudaGetDevice(&prev));
+  std::lock_guard<std::mutex> lk(g_arena_mu);
+  for (auto& kv : g_parked) {
+    LMVN_CUDA_TRY(cudaSetDevice(kv.first));
+    for (auto& a : kv.second) LMVN_CUDA_TRY(cudaMemset(a.p, byte, a.bytes));
+    LMVN_CUDA_TRY(cudaDeviceSynchronize());
+  }
+  LMVN_CUDA_TRY(cudaSetDevice(prev));
+  return 0;
+}
+
 Deconv::~Deconv() {
   if (arena || stream) cudaSetDevice(device);
   if (stream) cudaStreamSynchronize(stream);

@@ -195,6 +195,7 @@ struct Deconv {
 };
 
 void release_cached_memory();  // frees the arenas parked by destroyed handles
+int debug_fill_parked_arenas(int byte);  // memsets every parked arena (tests: the next handle starts on dirty memory)
 int resolve_device(int device);  // < 0 -> highest compute capability; validates range
 
 // debug hooks / legacy single-step entry points (host pointers unless noted)
