@@ -32,6 +32,12 @@ enum lmvn_strategy {
   LMVN_STRATEGY_GENERIC = 1, /* any shape: five separable passes per convolution             */
   LMVN_STRATEGY_FUSED = 2    /* three fused passes per convolution (power-of-two extents)    */
 };
+/* Extent limits.  The fused path takes power-of-two extents up to 1024 per axis (x >= 64, y and z >= 16); periodic
+ * embedding (lmvn_plan_create_embedded, AUTO one-shot calls) needs image + kernel - 1 <= 1024 on every axis.  Every
+ * other stack runs on the generic passes, which transform one axis line in shared memory (16 n bytes, at most
+ * 200 KB): they take at most 12800 points per axis (LMVN_MAX_GENERIC_AXIS).  A plan, padded plan or one-shot call
+ * with a longer axis (after padding) fails with "axis length N exceeds the shared-memory transform limit". */
+#define LMVN_MAX_GENERIC_AXIS 12800
 
 typedef struct lmvn_plan_info {
   int dims[3];

@@ -5,6 +5,7 @@
 
 #include <algorithm>
 #include <atomic>
+#include <cassert>
 #ifdef _OPENMP
 #include <omp.h>
 #endif
@@ -95,15 +96,26 @@ int resolve_device(int device) {
 // ------------------------------------------------------------------------------
 // plan store
 // ------------------------------------------------------------------------------
+// Every generic pass holds two n x L complex buffers in shared memory (L = clamp(2048 / n, 1, 32) lines per block):
+// 16 n L bytes, so 16 n bytes for n > 2048 whatever L is.  An axis longer than kMaxSmem / 16 = 12800 points cannot
+// be planned.
+static const size_t kMaxSmem = 200 * 1024;
+// radices of the longest factorisation of a length <= 12800 (3^8 = 6561, 2^2 3^7, 2^4 3^6, ...)
+static const int kMaxFactors = 8;
+
 static void factorize(int n, gen::AxisPlan& P) {
   P.n = n;
   P.nf = 0;
   int m = n;
-  while (m % 4 == 0) { P.factors[P.nf++] = 4; m /= 4; }
-  while (m % 2 == 0) { P.factors[P.nf++] = 2; m /= 2; }
-  for (int p = 3; p * p <= m; p += 2)
-    while (m % p == 0) { P.factors[P.nf++] = p; m /= p; }
-  if (m > 1) P.factors[P.nf++] = m;
+  auto push = [&](int r) {
+    assert(P.nf < kMaxFactors);
+    P.factors[P.nf++] = r;
+  };
+  while (m % 4 == 0) { push(4); m /= 4; }
+  while (m % 2 == 0) { push(2); m /= 2; }
+  for (int p = 3; p <= m / p; p += 2)
+    while (m % p == 0) { push(p); m /= p; }
+  if (m > 1) push(m);
 }
 
 FftPlan::~FftPlan() {
@@ -111,9 +123,18 @@ FftPlan::~FftPlan() {
     if (d_tw[a]) cudaFree(d_tw[a]);
 }
 
-static const size_t kMaxSmem = 200 * 1024;
-
 static int build_axis(FftPlan& fp, int a, int n) {
+  int L = 2048 / n;
+  if (L < 1) L = 1;
+  if (L > 32) L = 32;
+  const size_t smem = size_t(2) * n * L * sizeof(cplx);
+  // before the factorisation and the n-entry twiddle tables: a doomed plan allocates nothing
+  if (smem > kMaxSmem) {
+    set_last_error("axis length %d exceeds the shared-memory transform limit", n);
+    return -1;
+  }
+  fp.lines[a] = L;
+  fp.smem[a] = smem;
   factorize(n, fp.ax[a]);
   std::vector<cplx> tw(n);
   for (int k = 0; k < n; ++k) {
@@ -123,15 +144,6 @@ static int build_axis(FftPlan& fp, int a, int n) {
   LMVN_CUDA_TRY(cudaMalloc(reinterpret_cast<void**>(&fp.d_tw[a]), sizeof(cplx) * n));
   LMVN_CUDA_TRY(cudaMemcpy(fp.d_tw[a], tw.data(), sizeof(cplx) * n, cudaMemcpyHostToDevice));
   fp.ax[a].tw = fp.d_tw[a];
-  int L = 2048 / n;
-  if (L < 1) L = 1;
-  if (L > 32) L = 32;
-  fp.lines[a] = L;
-  fp.smem[a] = size_t(2) * n * L * sizeof(cplx);
-  if (fp.smem[a] > kMaxSmem) {
-    set_last_error("axis length %d exceeds the shared-memory transform limit", n);
-    return -1;
-  }
   return 0;
 }
 

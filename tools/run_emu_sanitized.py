@@ -39,4 +39,4 @@ _build.build_emu = lambda force=False, asan=False, ubsan=False: _path  # the fix
 import pytest  # noqa: E402
 
 sys.exit(pytest.main(["-x", "-q", "-m", "not gpu", "tests/test_emu_parity.py", "tests/test_slabs_emu.py",
-                      "tests/test_call_history.py"] + args))
+                      "tests/test_call_history.py", "tests/test_generic_extents.py"] + args))
